@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the B200-native PIN-SLAM hot path (contract: see the task statement / DESIGN.md §4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload at N=1: BASELINE.json configs[1] -- the fused kNN + SDF-MLP query (K1) over a batch of
 200 000 query points, K=8 neighbours, 32-d features, 2x64 decoder, C=33 probe cells, with the
@@ -396,6 +396,19 @@ def mapper_benchmark(args, standalone=True):
     return res
 
 
+def dump_outputs(path, out):
+    """The K1 output tensors as <path>/<name>.npy: floating outputs in float32, integer ones (nn_count) in float64
+    (exact); scratch buffers (names starting with "_") are not outputs."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, t in sorted(out.items()):
+        if name.startswith("_"):
+            continue
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -412,7 +425,13 @@ def main():
                          "configuration every committed number refers to")
     ap.add_argument("--workload", default="query", choices=["query", "mapper"],
                     help="query = BASELINE configs[1] (default, the headline); mapper = configs[4] data-parallel training")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="query workload: write what the last timed step returned (sdf, grad, sdf_std, certainty, "
+                         "nn_count of all 200 000 queries, ~6 MB) as DIR/<name>.npy; the inputs are seeded, so runs "
+                         "with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "query"):
+        ap.error("--dump-outputs writes the outputs of the query workload of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     global MAP_SCALE
     MAP_SCALE = float(args.map_scale)
@@ -478,6 +497,8 @@ def main():
     launches = ops.launch_count() - launches0
     total_ms = sum(step_ms)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
 
     # ---- end to end through the public call with host buffers
     q_host = q.cpu().pin_memory()
@@ -591,7 +612,7 @@ def main():
         del flush
         torch.cuda.empty_cache()
         try:
-            md = mapper_benchmark(argparse.Namespace(steps=max(20, args.steps), warmup=args.warmup), standalone=False)
+            md = mapper_benchmark(argparse.Namespace(steps=args.steps, warmup=args.warmup), standalone=False)
             if line is not None:
                 line["mapper_dp"] = {"ms_per_iter": md["ms_per_step"], "samples_per_s": md["value"],
                                      "allreduce_bytes": 4 * md["config"]["allreduce_floats"],
